@@ -269,9 +269,8 @@ _REF_IDCT = os.path.join(_HERE, "_ref", "libidct_ref.so")
 
 
 def idct_ref_available() -> bool:
-    """oracle/_ref/libidct_ref.so = /root/reference/c_components/lib/codecs_jpeg_idct_fast.c compiled as it is (oracle/Makefile)."""
-    if not os.path.exists(_REF_IDCT) and os.path.exists("/root/reference/c_components/lib/codecs_jpeg_idct_fast.c"):
-        subprocess.call(["make", "-C", _HERE, "-s", "CC=gcc", "ref"], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL)
+    """oracle/_ref/libidct_ref.so = the reference's c_components/lib/codecs_jpeg_idct_fast.c compiled as it is (oracle/Makefile,
+    run by __graft_entry__.build() where the reference tree is readable)."""
     return os.path.exists(_REF_IDCT)
 
 
